@@ -2,7 +2,7 @@
 """bench.py — gates/sec on BASELINE.json's workloads + Apply2x2 HBM roofline (contract: see DESIGN.md §Measurement).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload htcnot|qft|qv|grover]
-                  [--qubits n] [--depth d] [--precision 32|64]
+                  [--qubits n] [--depth d] [--precision 32|64] [--dump-outputs DIR]
 
 A "step" = one replay of the whole seeded circuit on a state vector that is already resident in HBM.  Default workload =
 BASELINE configs[1]: 30 qubits, H/T/CNOT depth 40, 1800 gates, fp32.  Other BASELINE configs: `--workload qft --precision 64`
@@ -13,6 +13,8 @@ of per-qubit probabilities inside the timed region.  `check` = self-checks compu
 (norm, mirror-circuit return probability, Grover success law): a throughput number over an unverified state is not a result.
 `--impl reference` times the compiled reference QEngineCPU (oracle/_ref) — or the oracle port when that binary did not
 travel — on a bounded, fixed sample of the same workload on the host cores.
+`--dump-outputs DIR` (1 GPU) writes what the last timed steps computed, for comparing two builds output for output:
+DIR/state_sample.npy = a fixed sample of the final state (see state_sample), DIR/qubit_probs.npy = Prob(q) of every qubit.
 """
 import argparse
 import json
@@ -146,6 +148,19 @@ def fused_single_qubit_sweep_probe(q, n, amp_bytes, peak, reps=5, warm=2):
         return {"error": repr(e)[:200]}
 
 
+def state_sample(q, n, page=1 << 12, pages=1 << 8):
+    """A fixed sample of the state, the same for every run at this n: the whole state up to page * pages amplitudes, else
+    `pages` pages of `page` amplitudes at seeded offsets.  -> float array (amplitudes, 2) of (real, imaginary) in the engine's
+    precision: 8 MiB (fp32) / 16 MiB (fp64) at most."""
+    import numpy as np
+    if (1 << n) <= page * pages:
+        spans = [(0, 1 << n)]
+    else:
+        spans = [(p * page, page) for p in sorted(random.Random(0).sample(range((1 << n) // page), pages))]
+    amps = np.concatenate([q.GetAmplitudePage(o, k) for o, k in spans])
+    return np.stack([amps.real, amps.imag], axis=-1)
+
+
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -276,7 +291,13 @@ def main():
                     help="N>1: qubit exchange by the fused NVLink peer-store kernel (default) or NCCL all_to_all + local swaps")
     ap.add_argument("--workload", default="htcnot", choices=["htcnot", "qft", "qv", "grover"],
                     help="htcnot = BASELINE configs[1] (default, the headline); qft = configs[2]; qv = configs[3]; grover = configs[4]")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed steps to DIR/<name>.npy (1 GPU, --impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus > 1):
+        ap.error("--dump-outputs needs --impl b200 on 1 GPU")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     world_req = max(1, args.gpus)
@@ -384,6 +405,7 @@ def main():
     stats = {k: stats1[k] - stats0.get(k, 0) for k in stats1}
     exchanges = (q.be.exchanges - ex0) if sharded else 0
     carried = (getattr(q.be, "carried_ops", 0) - car0) if sharded else 0
+    dumped_state = state_sample(q, n) if args.dump_outputs else None
     # ---- end-to-end arm: public API, host submission + init + result read inside the timed region -----------
     h2d = gates * (8 * 8 + 8 * 4)  # per gate: 8 doubles of matrix + offsets/powers words crossing the C ABI
     d2h = n * 8
@@ -509,6 +531,11 @@ def main():
         if world == 1 and not args.skip_cpu_baseline:
             cb = cpu_reference_sample(text, n, prec, args.cpu_sample_gates, 1, desc)
             line["cpu_baseline"] = {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample")}
+        if args.dump_outputs:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "state_sample.npy"), dumped_state)
+            np.save(os.path.join(args.dump_outputs, "qubit_probs.npy"), np.asarray(probs, dtype=np.float64))
         print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

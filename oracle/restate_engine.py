@@ -9,6 +9,7 @@ from __future__ import annotations
 import ctypes
 import os
 import subprocess
+import tempfile
 from ctypes import POINTER, c_double, c_int, c_uint64, c_void_p
 
 import numpy as np
@@ -21,18 +22,21 @@ _lib = None
 
 
 def build_restatement(force: bool = False) -> str:
+    """Compile liboracle_restate.so next to its sources when it is missing or older than they are; in a temporary directory
+    when the tree is read-only (bench.py's baseline leg may run from one)."""
     src = [os.path.join(_HERE, f) for f in ("qengine_restate.c", "qengine_restate_impl.h", "qalu_restate_impl.h")]
-    if force or not os.path.exists(_LIB) or os.path.getmtime(_LIB) < max(os.path.getmtime(s) for s in src):
-        subprocess.run(["gcc", "-O2", "-std=c11", "-fPIC", "-shared", "-fno-fast-math", "-ffp-contract=off", src[0], "-lm",
-                        "-o", _LIB], check=True)
-    return _LIB
+    if not force and os.path.exists(_LIB) and os.path.getmtime(_LIB) >= max(os.path.getmtime(s) for s in src):
+        return _LIB
+    out = _LIB if os.access(_HERE, os.W_OK) else os.path.join(tempfile.mkdtemp(prefix="oracle_restate_"), os.path.basename(_LIB))
+    subprocess.run(["gcc", "-O2", "-std=c11", "-fPIC", "-shared", "-fno-fast-math", "-ffp-contract=off", src[0], "-lm",
+                    "-o", out], check=True)
+    return out
 
 
 def _load():
     global _lib
     if _lib is None:
-        build_restatement()
-        _lib = ctypes.CDLL(_LIB)
+        _lib = ctypes.CDLL(build_restatement())
         for suf in ("_f32", "_f64"):
             for name in ("orc_prob_mask", "orc_prob_parity", "orc_collapse_parity", "orc_norm", "orc_expectation"):
                 getattr(_lib, name + suf).restype = c_double

@@ -1,7 +1,8 @@
 """Generate the committed golden fixtures from the UNMODIFIED reference (oracle/_ref/ref_harness_f{32,64}, i.e.
-Qrack::QEngineCPU compiled from /root/reference by oracle/Makefile).  Run in the build container only:
+Qrack::QEngineCPU compiled from the reference sources by oracle/Makefile, REF=<reference checkout>):
 
     make -C oracle ref && python tests/golden/make_golden.py
+    python tests/golden/make_golden.py reference [case ...]     # only the sampled outputs under reference/
 
 Each fixture = <name>.qs (the script) + <name>.f32.npz / <name>.f64.npz (final state of every register and the
 query results, as produced by the reference).  Scripts are deterministic (seeded python RNG).
@@ -220,6 +221,94 @@ SCRIPTS = {
 }
 
 
+def _harness(prec, text, td, *args):
+    """Run `text` on the compiled reference, outputs inside td."""
+    path = os.path.join(td, "c.qs")
+    with open(path, "w") as f:
+        f.write(text)
+    subprocess.run([os.path.join(ROOT, "oracle", "_ref", "ref_harness_f%d" % prec), path] + list(args), check=True)
+
+
+# Reference outputs kept under reference/ for the tests that compare with the reference on circuits too large for a
+# full-state fixture.  A state keeps a seeded sample of SAMPLE amplitudes of register 0 (the whole state when it is smaller).
+SAMPLE = 1024
+
+
+def state_case(text, prec, engine="cpu"):
+    dt = np.complex64 if prec == 32 else np.complex128
+    with tempfile.TemporaryDirectory() as td:
+        _harness(prec, text, td, "--dump", os.path.join(td, "s"), "--engine", engine)
+        st = np.fromfile(os.path.join(td, "s.0.bin"), dtype=dt)
+    idx = np.arange(st.size) if st.size <= SAMPLE else np.sort(np.random.default_rng(1).choice(st.size, SAMPLE, replace=False))
+    return {"text": text, "idx": idx.astype(np.int64), "amp": st[idx]}
+
+
+def results_case(text, prec):
+    """Query results of the fp`prec` reference; for fp32 also those of the fp64 build on the same circuit ("results_f64"):
+    the fp32 reference sums each Prob in fp32 per worker thread with a dynamic work split, so its own Prob wanders by up to
+    ~1e-4 from run to run at these sizes, and the tests take the probabilities from the fp64 build."""
+    out = {"text": text}
+    for p in ((32, 64) if prec == 32 else (64,)):
+        with tempfile.TemporaryDirectory() as td:
+            _harness(p, text, td, "--results", os.path.join(td, "r.txt"))
+            out["results" if p == prec else "results_f64"] = open(os.path.join(td, "r.txt")).read()
+    return out
+
+
+def full_size_text(n, kind):
+    """tests/test_parity_gpu.py::test_full_size_parity_against_the_compiled_reference: 30-qubit fp32 depth-2 H/T/CNOT or
+    29-qubit fp64 QFT prefix, then every per-qubit Prob and 64 sampled amplitudes."""
+    rng = random.Random(77)
+    if kind == "htcnot":
+        text = qscript.random_htcnot(n, 2, seed=31, timed=False)
+    else:
+        # H on a random half of the qubits, then the first 3 target qubits of QFT(0, n): 3 H + 84 controlled phases on all qubits
+        lines = ["qubits %d" % n] + ["H %d" % q for q in range(n) if rng.random() < 0.5]
+        for i in range(3):
+            hb = n - 1 - i
+            lines.append("H %d" % hb)
+            for j in range(hb):
+                lines.append("CPhaseRootN %d %d %d" % (hb - j + 1, j, hb))
+        text = "\n".join(lines) + "\n"
+    idx = sorted(rng.randrange(1 << n) for _ in range(64))
+    return text + "".join("Prob %d\n" % q for q in range(n)) + "".join("GetAmplitude %d\n" % i for i in idx)
+
+
+def sharded_26q_text(kind):
+    """tests/test_sharded_gpu.py::test_sharded_26q_against_the_compiled_reference: all per-qubit Prob, 48 sampled amplitudes."""
+    n = 26
+    rng = random.Random(5)
+    text = {"htcnot": lambda: qscript.random_htcnot(n, 6, seed=12, timed=False),
+            "qv": lambda: qscript.quantum_volume(n, depth=4, seed=13, timed=False),
+            "grover": lambda: "\n".join(l for l in qscript.grover(n, 1, target=3, timed=False).splitlines() if not l.startswith("ProbAll")) + "\n"}[kind]()
+    idx = sorted(rng.randrange(1 << n) for _ in range(48)) + [3]
+    return text + "".join("Prob %d\n" % q for q in range(n)) + "".join("GetAmplitude %d\n" % i for i in idx)
+
+
+C1_16Q = qscript.random_htcnot(16, 40, seed=20250921, timed=False)   # BASELINE configs[0] at reduced width
+C1_20Q = qscript.random_htcnot(20, 40, seed=20250921, timed=False)   # BASELINE configs[0]
+REFERENCE_CASES = {
+    "c1_16q_f32": lambda: state_case(C1_16Q, 32),
+    "c1_16q_f64": lambda: state_case(C1_16Q, 64),
+    # QPager over QEngineCPU with forced small pages (2^7 amplitudes)
+    "pager_10q_f32": lambda: state_case(qscript.random_htcnot(10, 6, seed=3, timed=False), 32, engine="pager:7"),
+    "c1_20q_f32": lambda: state_case(C1_20Q, 32),
+    "c1_20q_f64": lambda: state_case(C1_20Q, 64),
+    "full_30q_htcnot_f32": lambda: results_case(full_size_text(30, "htcnot"), 32),
+    "full_29q_qft_f64": lambda: results_case(full_size_text(29, "qft"), 64),
+    "sharded_26q_htcnot_f32": lambda: results_case(sharded_26q_text("htcnot"), 32),
+    "sharded_26q_qv_f32": lambda: results_case(sharded_26q_text("qv"), 32),
+    "sharded_26q_grover_f32": lambda: results_case(sharded_26q_text("grover"), 32),
+}
+
+
+def main_reference(names):
+    os.makedirs(os.path.join(HERE, "reference"), exist_ok=True)
+    for name in names or REFERENCE_CASES:
+        np.savez_compressed(os.path.join(HERE, "reference", name + ".npz"), **REFERENCE_CASES[name]())
+        print("wrote reference/%s.npz" % name)
+
+
 def main():
     for name, text in SCRIPTS.items():
         path = os.path.join(HERE, name + ".qs")
@@ -241,4 +330,7 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:2] == ["reference"]:
+        main_reference(sys.argv[2:])
+    else:
+        main()

@@ -72,14 +72,14 @@ def test_b200_arm_other_baseline_workloads(workload, extra):
 
 
 def test_reference_arm_runs_on_host_cores():
-    if util.ref_harness(32) is None:
-        pytest.skip("oracle/_ref not built")
+    # the compiled reference when oracle/_ref was built (it needs the reference sources), otherwise the oracle port
+    kind = "port" if util.ref_harness(32) is None else "reference"
     r = subprocess.run([sys.executable, os.path.join(util.ROOT, "bench.py"), "--impl", "reference", "--qubits", "16", "--steps", "2",
                         "--warmup", "1"], capture_output=True, text=True, timeout=600, cwd=util.ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     j = _last_json(r.stdout)
     assert j["impl"] == "reference" and j["unit"] == "gates/s" and j["value"] > 0
-    assert j["cpu_baseline"]["kind"] == "reference" and j["cpu_baseline"]["cores"] >= 1
+    assert j["cpu_baseline"]["kind"] == kind and j["cpu_baseline"]["cores"] >= 1
     assert j["e2e"]["h2d_bytes_per_step"] == 0 and j["e2e"]["d2h_bytes_per_step"] == 0
     # the sample is a fixed prefix of the circuit (>= one full layer incl. CNOTs), whatever --steps is, and `config` is the b200 arm's
     assert j["reference_sample"]["ops_total"] >= 60 and len(j["reference_sample"]["segment_seconds"]) == 2
@@ -93,3 +93,47 @@ def test_reference_arm_runs_on_host_cores():
     r = subprocess.run([sys.executable, os.path.join(util.ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--qubits", "16"],
                        capture_output=True, text=True, timeout=120, cwd=util.ROOT, env=env)
     assert r.returncode == 0 and not r.stdout.strip()
+
+
+def test_dump_outputs_are_the_same_from_run_to_run(tmp_path):
+    """--dump-outputs DIR: the last timed step's state sample and the per-qubit probabilities, in the engine's precision, identical
+    for two runs with the same arguments."""
+    import numpy as np
+    outs = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        shim = (SHIM % util.ROOT).replace("'--skip-cpu-baseline']", "'--skip-cpu-baseline', '--dump-outputs', %r]" % str(d))
+        r = subprocess.run([sys.executable, "-c", shim], capture_output=True, text=True, timeout=600, cwd=util.ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        outs.append({f.name: np.load(str(f)) for f in d.iterdir()})
+    a, b = outs
+    assert set(a) == {"state_sample.npy", "qubit_probs.npy"}
+    assert a["state_sample.npy"].dtype == np.float32 and a["state_sample.npy"].shape == (1 << 9, 2)
+    assert a["qubit_probs.npy"].dtype == np.float64 and a["qubit_probs.npy"].shape == (9,)
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+    # the state sample is the state: its marginals are the probabilities the end-to-end arm read
+    st = a["state_sample.npy"].astype(np.float64)
+    p = st[:, 0] ** 2 + st[:, 1] ** 2
+    idx = np.arange(p.size)
+    assert np.allclose([p[(idx >> q) & 1 == 1].sum() for q in range(9)], a["qubit_probs.npy"], atol=1e-5)
+
+
+def test_state_sample_pages_are_fixed_and_exact():
+    import numpy as np
+    import bench
+
+    class Engine:
+        def __init__(self, n):
+            self.st = (np.arange(1 << n) * (1 + 2j)).astype(np.complex128)
+
+        def GetAmplitudePage(self, offset, length):
+            return self.st[offset:offset + length]
+
+    n = 22
+    a, b = bench.state_sample(Engine(n), n), bench.state_sample(Engine(n), n)
+    assert a.dtype == np.float64 and a.shape == (1 << 20, 2) and np.array_equal(a, b)
+    pos = a[:, 0].astype(np.int64)              # amplitude i holds i + 2i j
+    assert np.array_equal(a[:, 1], 2 * a[:, 0]) and np.all(np.diff(pos) > 0)
+    assert np.all(pos.reshape(-1, 1 << 12) % (1 << 12) == np.arange(1 << 12))   # whole pages
+    assert pos.max() >= (1 << 21)                                                # spread over the state

@@ -1,7 +1,7 @@
 """GPU parity tests proper: the CUDA path (through the C ABI, libb200sv.so) against
  (1) the committed golden fixtures produced by the unmodified reference QEngineCPU,
  (2) the oracle restatement on fresh seeded circuits at sizes it finishes in seconds,
- (3) the compiled reference itself (oracle/_ref/ref_harness_*) when it travelled to the box,
+ (3) what the compiled reference produced on larger circuits, stored under tests/golden/reference,
  (4) size-independent properties at BASELINE.json's full sizes (28-30 qubits).
 Tolerances (north_star): max |delta amp| <= 1e-6 (fp32) / 1e-12 (fp64)."""
 import os
@@ -53,12 +53,11 @@ def test_c1_20q_vs_oracle(prec, fusion):
 
 @pytest.mark.parametrize("prec", [32, 64])
 def test_c1_20q_vs_compiled_reference(prec):
-    if util.ref_harness(prec) is None:
-        pytest.skip("oracle/_ref not present on this box")
-    text = qscript.random_htcnot(20, 40, seed=20250921, timed=False)
-    want, _ = util.run_reference(text, prec)
-    got, _ = run_cuda(text, prec, 1)
-    util.assert_states_close(got, want, prec, "C1-ref")
+    """BASELINE configs[0] against the compiled reference's final state (stored sample, tests/golden/reference)."""
+    ref = util.load_reference("c1_20q_f%d" % prec)
+    assert ref["text"] == qscript.random_htcnot(20, 40, seed=20250921, timed=False)
+    got, _ = run_cuda(ref["text"], prec, 1)
+    util.assert_sample_close(got[0], ref, prec, "C1-ref")
 
 
 @pytest.mark.parametrize("fusion", [0, 1])
@@ -313,38 +312,18 @@ def test_full_size_mirror_circuit_and_norm(n, prec):
 
 
 @pytest.mark.parametrize("n,prec,kind", [(30, 32, "htcnot"), (29, 64, "qft")])
-def test_full_size_parity_against_the_compiled_reference(n, prec, kind, tmp_path):
+def test_full_size_parity_against_the_compiled_reference(n, prec, kind):
     """Full-width states against the REFERENCE, not against ourselves: a 30-qubit fp32 depth-2 H/T/CNOT circuit (90 gates) and a
     29-qubit fp64 QFT prefix (same bytes) are replayed on the compiled reference QEngineCPU (oracle/_ref, host cores) and on the
-    CUDA engine; every per-qubit Prob and 64 sampled amplitudes must agree (1e-6 fp32 / 1e-12 fp64 on amplitudes)."""
-    if util.ref_harness(prec) is None:
-        pytest.skip("oracle/_ref not built")
-    rng = random.Random(77)
-    if kind == "htcnot":
-        text = qscript.random_htcnot(n, 2, seed=31, timed=False)
-    else:
-        # H on a random half of the qubits, then the first 3 target qubits of QFT(0, n): 3 H + 84 controlled phases on all qubits
-        lines = ["qubits %d" % n] + ["H %d" % q for q in range(n) if rng.random() < 0.5]
-        for i in range(3):
-            hb = n - 1 - i
-            lines.append("H %d" % hb)
-            for j in range(hb):
-                lines.append("CPhaseRootN %d %d %d" % (hb - j + 1, j, hb))
-        text = "\n".join(lines) + "\n"
-    idx = sorted(rng.randrange(1 << n) for _ in range(64))
-    text += "".join("Prob %d\n" % q for q in range(n)) + "".join("GetAmplitude %d\n" % i for i in idx)
-    import subprocess
-    sp = tmp_path / "full.qs"
-    sp.write_text(text)
-    subprocess.run([util.ref_harness(prec), str(sp), "--results", str(tmp_path / "r.txt")], check=True, timeout=1500)
-    want = qscript.parse_results(open(str(tmp_path / "r.txt")).read())
+    CUDA engine; every per-qubit Prob and 64 sampled amplitudes must agree (1e-6 fp32 / 1e-12 fp64 on amplitudes).  The circuits and
+    the reference's results are stored in tests/golden/reference (make_golden.py full_size_text)."""
+    ref = util.load_reference("full_%dq_%s_f%d" % (n, kind, prec))
+    text = ref["text"]
+    want = qscript.parse_results(ref["results"])
     # the fp32 reference sums each Prob (2^29 terms) in fp32 per worker thread with a dynamic work split, so its own value wanders by
     # up to ~1e-4 from run to run (measured: 9e-5 between two runs at 24 qubits): the per-qubit probabilities of the fp32 case are
     # taken from the fp64 build of the reference on the same circuit
-    want_prob = want
-    if prec == 32 and util.ref_harness(64) is not None:
-        subprocess.run([util.ref_harness(64), str(sp), "--results", str(tmp_path / "r64.txt")], check=True, timeout=1500)
-        want_prob = qscript.parse_results(open(str(tmp_path / "r64.txt")).read())
+    want_prob = qscript.parse_results(ref["results_f64"]) if prec == 32 else want
     _, got = qscript.run(text, util.make_factory(QEngineCUDA, prec))
     assert len(got) == len(want) == n + 64
     worst_p = worst_a = 0.0

@@ -107,29 +107,19 @@ def _worker_queries(rank, world, port, text, prec, out_path):
 @pytest.mark.parametrize("kind", ["htcnot", "qv", "grover"])
 def test_sharded_26q_against_the_compiled_reference(kind, tmp_path):
     """BASELINE.md §3 'Parity': the sharded path at 26 qubits over every GPU of the box (8 ranks on the 8-GPU box) against the
-    compiled reference QEngineCPU: all per-qubit Prob, 48 sampled amplitudes (1e-6), the norm, and a sharded MAll."""
+    compiled reference QEngineCPU: all per-qubit Prob, 48 sampled amplitudes (1e-6), the norm, and a sharded MAll.  The circuits and
+    the reference's results are stored in tests/golden/reference (make_golden.py sharded_26q_text)."""
     ng = _ngpu()
-    if ng < 2 or util.ref_harness(32) is None:
-        pytest.skip("needs >= 2 GPUs and oracle/_ref")
+    if ng < 2:
+        pytest.skip("needs >= 2 GPUs")
     world = 8 if ng >= 8 else (4 if ng >= 4 else 2)
     n = 26
-    rng = random.Random(5)
-    text = {"htcnot": lambda: qscript.random_htcnot(n, 6, seed=12, timed=False),
-            "qv": lambda: qscript.quantum_volume(n, depth=4, seed=13, timed=False),
-            "grover": lambda: "\n".join(l for l in qscript.grover(n, 1, target=3, timed=False).splitlines() if not l.startswith("ProbAll")) + "\n"}[kind]()
-    idx = sorted(rng.randrange(1 << n) for _ in range(48)) + [3]
-    text += "".join("Prob %d\n" % q for q in range(n)) + "".join("GetAmplitude %d\n" % i for i in idx)
-    import subprocess
-    sp = tmp_path / "s.qs"
-    sp.write_text(text)
-    subprocess.run([util.ref_harness(32), str(sp), "--results", str(tmp_path / "r.txt")], check=True, timeout=1200)
-    want = np.array([v for _, vals in qscript.parse_results(open(str(tmp_path / "r.txt")).read()) for v in vals], dtype=np.float64)
+    ref = util.load_reference("sharded_26q_%s_f32" % kind)
+    text = ref["text"]
+    want = np.array([v for _, vals in qscript.parse_results(ref["results"]) for v in vals], dtype=np.float64)
     # the fp32 reference sums each Prob (2^25 terms) in fp32 per worker thread with a dynamic work split: its own value wanders by
     # ~1e-4 from run to run.  The per-qubit probabilities are therefore taken from the fp64 build of the reference (same circuit).
-    want_p = want[:n]
-    if util.ref_harness(64) is not None:
-        subprocess.run([util.ref_harness(64), str(sp), "--results", str(tmp_path / "r64.txt")], check=True, timeout=1200)
-        want_p = np.array([v for _, vals in qscript.parse_results(open(str(tmp_path / "r64.txt")).read()) for v in vals], dtype=np.float64)[:n]
+    want_p = np.array([v for _, vals in qscript.parse_results(ref["results_f64"]) for v in vals], dtype=np.float64)[:n]
     import torch.multiprocessing as mp
     out = str(tmp_path / "o.npz")
     for attempt in range(3):

@@ -1,8 +1,6 @@
 """Shared helpers for the parity tests (test infrastructure)."""
 import os
 import random
-import subprocess
-import tempfile
 
 import numpy as np
 
@@ -33,27 +31,24 @@ def load_golden(name, prec):
     return text, regs, results
 
 
+def load_reference(name):
+    """Stored outputs of the compiled reference (tests/golden/reference, written by make_golden.py): the script "text" and
+    either a seeded sample of register 0's final amplitudes ("idx", "amp") or the query results ("results", and "results_f64"
+    from the fp64 build for fp32 cases)."""
+    z = np.load(os.path.join(GOLDEN, "reference", name + ".npz"))
+    return {k: (str(z[k]) if z[k].dtype.kind == "U" else z[k]) for k in z.files}
+
+
+def assert_sample_close(state, ref, prec, what=""):
+    """register 0's state against the reference's stored amplitude sample"""
+    assert state.size > int(ref["idx"].max()), (what, state.size)
+    d = float(np.abs(state[ref["idx"]].astype(np.complex128) - ref["amp"].astype(np.complex128)).max())
+    assert d <= AMP_TOL[prec], "%s: max |delta amp| over %d sampled amplitudes = %.3e > %.1e" % (what, ref["idx"].size, d, AMP_TOL[prec])
+
+
 def ref_harness(prec):
     p = os.path.join(ROOT, "oracle", "_ref", "ref_harness_f%d" % prec)
     return p if os.path.exists(p) else None
-
-
-def run_reference(text, prec, engine="cpu"):
-    """Run a script on the compiled reference (oracle/_ref). Returns (regs, results)."""
-    h = ref_harness(prec)
-    assert h is not None
-    dt = np.complex64 if prec == 32 else np.complex128
-    with tempfile.TemporaryDirectory() as td:
-        sp = os.path.join(td, "c.qs")
-        open(sp, "w").write(text)
-        subprocess.run([h, sp, "--dump", os.path.join(td, "s"), "--results", os.path.join(td, "r.txt"), "--engine", engine],
-                       check=True)
-        regs = {}
-        for fn in os.listdir(td):
-            if fn.startswith("s.") and fn.endswith(".bin"):
-                regs[int(fn.split(".")[1])] = np.fromfile(os.path.join(td, fn), dtype=dt)
-        results = qscript.parse_results(open(os.path.join(td, "r.txt")).read())
-    return regs, results
 
 
 def make_factory(cls, prec, **kw):
